@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA engine (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N ...          # the reference's own CPU path (oracle/_ref), all host cores
+  python bench.py ... --dump-outputs DIR                  # also save what the last timed step computed (see dump_outputs)
 
 One "step" = one pass of the hot path over one batch of synthetic 48 kHz PCM already resident in HBM:
 65 536 mono frames of N=2048 per GPU, laid out as 4096 independent streams x 16 consecutive frames (hop = N)
@@ -244,6 +245,27 @@ def time_steps(torch, stream, step, steps, warmup):
     return [evs[k].elapsed_time(evs[k + 1]) for k in range(steps)]
 
 
+DUMP_BYTES = 48 << 20  # all ranks together: a dump stays well under 64 MB, so two builds can be compared output for output
+
+
+def dump_outputs(torch, out_dir, out, rank, world):
+    """Save the dB spectra the last timed step wrote ([streams, frames, 1, bins] float32) as db.npy, and the indices of the
+    streams saved as db_streams.npy (float64).  Each rank gets DUMP_BYTES / world; when its output is larger, a fixed seeded
+    sample of streams is saved, so the same arguments always select the same streams.  Ranks other than 0 add a _rank<r>
+    suffix."""
+    import numpy as np
+
+    S = out.shape[0]
+    n = min(S, max(1, DUMP_BYTES // world // (out[0].numel() * out.element_size())))
+    idx = np.arange(S) if n == S else np.sort(np.random.default_rng(0xB200).choice(S, n, replace=False))
+    sel = out.index_select(0, torch.as_tensor(idx, device=out.device)).cpu().numpy()
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    sfx = "" if rank == 0 else f"_rank{rank}"
+    np.save(d / f"db{sfx}.npy", sel)
+    np.save(d / f"db_streams{sfx}.npy", idx.astype(np.float64))
+
+
 def parity_subset(torch, device, pcm, S, T):
     """SURVEY §8(d): run the MEASURED launch geometry once from a fresh state and compare the first 256 frames of the
     shard plus streams from the far ends of the grid with the reference's generic CPU path (oracle/_ref; the C port if
@@ -430,6 +452,8 @@ def run_gpu_arm(args):
     total_ms = evs[0].elapsed_time(evs[-1])
     per_launch = [evs[k].elapsed_time(evs[k + 1]) for k in range(args.steps)]
     clocks = sampler.stop(t_begin, t_end) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, out, rank, world)
     ms_per_step = max_over_ranks(total_ms) / args.steps
     value = frames_per_gpu * world / (ms_per_step * 1e-3)
 
@@ -585,7 +609,10 @@ def main():
     ap.add_argument("--no-layouts", action="store_true")
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="save the spectra of the last timed step as .npy files in DIR")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs saves the GPU path's spectra; the reference arm only measures throughput")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

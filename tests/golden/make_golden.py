@@ -3,6 +3,7 @@
 (make -C oracle/ref_build).  Run in the dev container where /root/reference exists:
 
     python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --reference-outputs     # only the ref_*.npz files (see main_reference_outputs)
 
 Each case_*.npz holds: settings (json), channels, hop, pcm [cc, samples] float32, and what the reference's
 WAVSourceGeneric produced tick by tick: db [T, dch, B], points [T, dch, P] (generic interpolation path),
@@ -180,8 +181,29 @@ def main_stall():
         print("stall", name, "N", N, "skipped ticks", skipped, "db at first skipped tick: max", float(db[J].max()))
 
 
+# What the tests that compare with the reference on their own inputs need from it (test_oracle_vs_reference, test_wave,
+# test_meter, test_gpu_host): each of those modules builds its inputs and runs the reference in reference_records(); the
+# result goes to ref_<name>.npz, read back by helpers.ReferenceOutputs.
+REFERENCE_OUTPUTS = {"oracle_vs_reference": "test_oracle_vs_reference", "wave": "test_wave", "meter": "test_meter",
+                     "gpu_host": "test_gpu_host"}
+
+
+def main_reference_outputs():
+    import importlib
+
+    from helpers import ReferenceOutputs
+
+    for name, module in REFERENCE_OUTPUTS.items():
+        recs = importlib.import_module(module).reference_records()
+        ReferenceOutputs.save(name, recs)
+        print("reference outputs", name, len(recs), "cases", (OUT / f"ref_{name}.npz").stat().st_size, "bytes")
+
+
 if __name__ == "__main__":
     import sys
+    if "--reference-outputs" in sys.argv:
+        main_reference_outputs()
+        sys.exit(0)
     if "--stall-only" in sys.argv:
         main_stall()
         sys.exit(0)

@@ -1,9 +1,14 @@
 """Shared test helpers: synthetic PCM (SURVEY.md §8d) and the parity metric (DESIGN.md §Parity)."""
 from __future__ import annotations
 
+import hashlib
+import json
+from pathlib import Path
+
 import numpy as np
 
 SR = 48000
+GOLDEN = Path(__file__).resolve().parent / "golden"
 
 
 def synth_pcm(n_streams: int, channels: int, n_samples: int, seed: int = 0xB200, zero_frames=(), frame_len=0,
@@ -120,3 +125,69 @@ def fp64_truth_db(pcm, window, window_sum, n_frames, hop, g, db_min=-758.59564):
         with np.errstate(divide="ignore"):
             out[t] = np.where(state > 0, 20.0 * np.log10(np.maximum(state, 1e-300)), db_min)
     return out
+
+
+# ---- what the compiled reference produced, stored under tests/golden/ref_*.npz by make_golden.py --reference-outputs ----
+#
+# Arrays the tests compare bit for bit are stored as digests; arrays compared within a tolerance are stored as a fixed
+# sample of entries per row: the first and the last entry, the row's largest (so that a spectrum's frame peak is in its
+# sample) and k more drawn with a seed.  Only the values and the rows' peak positions are stored; the other positions
+# are drawn again when the sample is compared.
+
+def digest(a) -> str:
+    """Short content hash of an array (dtype, shape and bytes); "none" for None."""
+    if a is None:
+        return "none"
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()[:16]
+
+
+def sample_columns(n: int, peaks, k: int, seed: int) -> np.ndarray:
+    """[rows, k+3] positions of a sample of rows of n entries: 0, n-1, the row's peak, then k distinct positions."""
+    rng = np.random.default_rng(seed)
+    k = min(k, n)
+    return np.array([[0, n - 1, p, *rng.choice(n, k, replace=False)] for p in peaks], dtype=np.intp)
+
+
+def sample_rows(a, k: int, seed: int):
+    """(values [rows, k+3], record) of a sample of a[..., n] viewed as rows of n; the record (JSON-able) lets
+    take_sample() find the same positions again."""
+    rows = np.asarray(a).reshape(-1, a.shape[-1])
+    peaks = [int(i) for i in rows.argmax(axis=1)]
+    cols = sample_columns(rows.shape[1], peaks, k, seed)
+    return np.take_along_axis(rows, cols, axis=1), {"peaks": peaks, "k": k, "seed": seed, "cols": digest(cols)}
+
+
+def take_sample(a, record: dict) -> np.ndarray:
+    """The entries of a[..., n] at the positions of a sample_rows() sample, as [rows, k+3]."""
+    rows = np.asarray(a).reshape(-1, a.shape[-1])
+    cols = sample_columns(rows.shape[1], record["peaks"], record["k"], record["seed"])
+    assert digest(cols) == record["cols"], "the sampled positions differ from the stored ones"
+    return np.take_along_axis(rows, cols, axis=1)
+
+
+class ReferenceOutputs:
+    """tests/golden/ref_<name>.npz: per case, a JSON record (digests, scalars) and the sampled arrays "<case>__<key>"."""
+
+    def __init__(self, name: str):
+        self.path = GOLDEN / f"ref_{name}.npz"
+        z = np.load(self.path, allow_pickle=False)
+        self.meta = json.loads(str(z["meta"]))
+        self.arrays = {k: z[k] for k in z.files if k != "meta"}
+
+    def __getitem__(self, case: str) -> dict:
+        rec = dict(self.meta[case])
+        pre = case + "__"
+        rec.update({k[len(pre):]: v for k, v in self.arrays.items() if k.startswith(pre)})
+        return rec
+
+    @staticmethod
+    def save(name: str, records: dict):
+        """records: {case: {key: json-able value or np.ndarray}}; ndarrays go to their own members."""
+        meta, arrays = {}, {}
+        for case, rec in records.items():
+            meta[case] = {k: v for k, v in rec.items() if not isinstance(v, np.ndarray)}
+            arrays.update({f"{case}__{k}": v for k, v in rec.items() if isinstance(v, np.ndarray)})
+        np.savez_compressed(GOLDEN / f"ref_{name}.npz", meta=json.dumps(meta, sort_keys=True), **arrays)

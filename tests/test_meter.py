@@ -1,9 +1,9 @@
 """Level meter (tick_meter) and RMS feed (update_input_rms): SURVEY.md §8(f) rank 4 / §8(a) a9.
 
-CPU: the oracle restatement (oracle/wf_oracle_meter.c) bit-exact against the compiled reference and against the
-committed golden fixtures.  GPU: the CUDA path (wf_meter_* through the C-ABI) against the oracle — bit-exact for peak
-values and silent flags, 1e-5 relative for RMS values: an fp32 sum of W squares depends on the order of the additions —
-the reference's own AVX path (src/source_avx.cpp:257-268, 16 partial sums) differs from its generic path (ring order,
+CPU: the oracle restatement (oracle/wf_oracle_meter.c) bit-exact against what the compiled reference produced
+(tests/golden/ref_meter.npz, digests of every tick's values) and against the committed golden fixtures.  GPU: the CUDA
+path (wf_meter_* through the C-ABI) against the oracle — bit-exact for peak values and silent flags, 1e-5 relative for
+RMS values: an fp32 sum of W squares depends on the order of the additions — the reference's own AVX path (src/source_avx.cpp:257-268, 16 partial sums) differs from its generic path (ring order,
 one accumulator) by 1.8e-6 on this data; the CUDA path sums 256-sample blocks.
 """
 from __future__ import annotations
@@ -14,7 +14,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from helpers import synth_pcm
+from helpers import ReferenceOutputs, digest, synth_pcm
 
 GOLD = sorted((Path(__file__).parent / "golden").glob("meter_*.npz"))
 
@@ -35,34 +35,28 @@ def _case_pcm(ch, T, hop, S=1):
 
 # ---- CPU: oracle pinned to the reference -------------------------------------------------------------------------
 
+@pytest.fixture(scope="module")
+def ref():
+    return ReferenceOutputs("meter")
+
+
 @pytest.mark.parametrize("settings,ch,hop", METER_CASES)
-def test_meter_oracle_is_bit_exact_vs_compiled_reference(settings, ch, hop):
-    refbind = pytest.importorskip("oracle.refbind")
-    if not refbind.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+def test_meter_oracle_is_bit_exact_vs_compiled_reference(settings, ch, hop, ref):
     from oracle.oraclebind import OracleMeter
 
     T = 60
     pcm = _case_pcm(ch, T, hop)[0]
-    r = refbind.RefSource({"display_mode": "level_meter", **settings}, channels=ch)
-    ref = r.run_meter(pcm, T, hop)
+    rec = ref[f"case{METER_CASES.index((settings, ch, hop))}"]
+    assert digest(pcm) == rec["inputs"], "inputs differ from the ones the reference was run on"
     o = OracleMeter(settings, channels=ch)
-    assert o.window == r.fft_size
+    assert o.window == rec["window"]
     out = o.run(pcm, T, hop)
     for key in ("db", "lin", "silent"):
-        assert np.array_equal(ref[key], out[key]), key
-    assert ref["silent"].sum() > 0 or settings.get("floor", -65) < -60
+        assert digest(out[key]) == rec[key], key
+    assert out["silent"].sum() > 0 or settings.get("floor", -65) < -60
 
 
-@pytest.mark.parametrize("seed", range(30))
-def test_meter_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed):
-    """Differential fuzz of the level-meter oracle against the unmodified reference (generic path): random window, mode,
-    smoothing, gravity, floor, packet size and channel count, with a silent stretch."""
-    refbind = pytest.importorskip("oracle.refbind")
-    if not refbind.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    from oracle.oraclebind import OracleMeter
-
+def _random_case(seed):
     rng = np.random.default_rng(9000 + seed)
     ch = int(rng.choice([1, 2]))
     settings = {"meter_buf": int(rng.choice([5, 10, 20, 50, 100, 150, 300])), "rms_mode": bool(rng.uniform() < 0.5),
@@ -72,28 +66,55 @@ def test_meter_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed):
     hop = int(rng.choice([97, 441, 480, 800, 801, 1024, 1601]))
     T = 50
     pcm = _case_pcm(ch, T, hop)[0] * np.float32(rng.choice([1.0, 0.1, 0.01]))
-    r = refbind.RefSource({"display_mode": "level_meter", **settings}, channels=ch)
-    ref = r.run_meter(pcm, T, hop)
+    return settings, ch, hop, T, pcm
+
+
+@pytest.mark.parametrize("seed", range(30))
+def test_meter_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed, ref):
+    """Differential fuzz of the level-meter oracle against the unmodified reference (generic path): random window, mode,
+    smoothing, gravity, floor, packet size and channel count, with a silent stretch."""
+    from oracle.oraclebind import OracleMeter
+
+    settings, ch, hop, T, pcm = _random_case(seed)
+    rec = ref[f"random{seed}"]
+    assert digest(pcm) == rec["inputs"], "inputs differ from the ones the reference was run on"
     o = OracleMeter(settings, channels=ch)
-    assert o.window == r.fft_size
+    assert o.window == rec["window"]
     out = o.run(pcm, T, hop)
     for key in ("db", "lin", "silent"):
-        assert np.array_equal(ref[key], out[key]), (key, settings, hop)
+        assert digest(out[key]) == rec[key], (key, settings, hop)
 
 
 @pytest.mark.parametrize("ch", [1, 2])
-def test_rms_feed_oracle_is_bit_exact_vs_compiled_reference(ch):
-    refbind = pytest.importorskip("oracle.refbind")
-    if not refbind.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+def test_rms_feed_oracle_is_bit_exact_vs_compiled_reference(ch, ref):
     from oracle.oraclebind import OracleMeter
 
     T, hop = 90, 800
     pcm = _case_pcm(ch, T, hop)[0]
-    r = refbind.RefSource({"normalize_volume": True, "fft_size": 1024}, channels=ch)
-    ref = r.run_meter(pcm, T, hop)["rms"]
+    rec = ref[f"rms_feed{ch}"]
+    assert digest(pcm) == rec["inputs"], "inputs differ from the ones the reference was run on"
     out = OracleMeter({}, channels=ch).run(pcm, T, hop, meter=False, rms=True)["rms"]
-    assert np.array_equal(ref, out)
+    assert digest(out) == rec["rms"]
+
+
+def reference_records():
+    """What the compiled reference's tick_meter / update_input_rms (oracle/_ref) produced for each case above, as digests;
+    tests/golden/make_golden.py stores them."""
+    from oracle import refbind
+
+    recs = {}
+    cases = [(f"case{i}", (s, c, h, 60, _case_pcm(c, 60, h)[0])) for i, (s, c, h) in enumerate(METER_CASES)] \
+        + [(f"random{seed}", _random_case(seed)) for seed in range(30)]
+    for name, (settings, ch, hop, T, pcm) in cases:
+        r = refbind.RefSource({"display_mode": "level_meter", **settings}, channels=ch)
+        out = r.run_meter(pcm, T, hop)
+        recs[name] = {"inputs": digest(pcm), "window": r.fft_size, **{k: digest(out[k]) for k in ("db", "lin", "silent")}}
+    for ch in (1, 2):
+        T, hop = 90, 800
+        pcm = _case_pcm(ch, T, hop)[0]
+        r = refbind.RefSource({"normalize_volume": True, "fft_size": 1024}, channels=ch)
+        recs[f"rms_feed{ch}"] = {"inputs": digest(pcm), "rms": digest(r.run_meter(pcm, T, hop)["rms"])}
+    return recs
 
 
 @pytest.mark.parametrize("path", GOLD, ids=[p.stem for p in GOLD])

@@ -1,8 +1,8 @@
 """Waveform (oscilloscope) mode, tick_waveform: SURVEY.md §8(f) rank 4.
 
-CPU: the oracle restatement (oracle/wf_oracle_meter.c, wfo_wave_*) bit-exact against the compiled reference and against the
-committed golden fixtures.  GPU: the CUDA path (wf_wave_* through the C-ABI) against the oracle — which points are emitted and
-which sample each takes is integer arithmetic and must match exactly (checked through the DB_MIN pattern and the silent
+CPU: the oracle restatement (oracle/wf_oracle_meter.c, wfo_wave_*) bit-exact against what the compiled reference produced
+(tests/golden/ref_wave.npz, digests of every tick's output) and against the committed golden fixtures.  GPU: the CUDA
+path (wf_wave_* through the C-ABI) against the oracle — which points are emitted and which sample each takes is integer arithmetic and must match exactly (checked through the DB_MIN pattern and the silent
 flags); the dBFS values agree to 1e-4 dB (log10f last-bit differences between glibc and CUDA).
 """
 from __future__ import annotations
@@ -13,7 +13,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from helpers import synth_pcm
+from helpers import ReferenceOutputs, digest, synth_pcm
 
 GOLD = sorted((Path(__file__).parent / "golden").glob("wave_*.npz"))
 
@@ -37,31 +37,18 @@ def _case(settings, ch, hop, T=50, S=1):
     return pcm, rms
 
 
+@pytest.fixture(scope="module")
+def ref():
+    return ReferenceOutputs("wave")
+
+
 @pytest.mark.parametrize("settings,ch,hop", WAVE_CASES)
-def test_wave_oracle_is_bit_exact_vs_compiled_reference(settings, ch, hop):
-    refbind = pytest.importorskip("oracle.refbind")
-    if not refbind.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    from oracle.oraclebind import OracleWave
-
-    T = 50
-    pcm, rms = _case(settings, ch, hop, T)
-    r = refbind.RefSource({"display_mode": "waveform", **settings}, channels=ch)
-    ref = r.run_wave(pcm[0], T, hop, rms=None if rms is None else rms[0])
-    out = OracleWave(settings, channels=ch).run(pcm[0], T, hop, rms=None if rms is None else rms[0])
-    assert np.array_equal(ref["out"], out["out"])
-    assert np.array_equal(ref["silent"], out["silent"])
+def test_wave_oracle_is_bit_exact_vs_compiled_reference(settings, ch, hop, ref):
+    rec = ref[f"case{WAVE_CASES.index((settings, ch, hop))}"]
+    _check_bit_exact(rec, settings, ch, hop, *_case(settings, ch, hop, T=50))
 
 
-@pytest.mark.parametrize("seed", range(30))
-def test_wave_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed):
-    """Differential fuzz of the waveform-mode oracle against the unmodified reference: random width, window length, packet size,
-    channel layout, volume normalisation, stretches of zeros and of full-scale samples (the all-zero silent rule's raw material)."""
-    refbind = pytest.importorskip("oracle.refbind")
-    if not refbind.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    from oracle.oraclebind import OracleWave
-
+def _random_case(seed):
     rng = np.random.default_rng(7000 + seed)
     ch = int(rng.choice([1, 2]))
     settings = {"width": int(rng.choice([64, 200, 301, 640, 800, 1000, 1920])), "meter_buf": int(rng.choice([5, 10, 20, 50, 150, 500]))}
@@ -78,11 +65,39 @@ def test_wave_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed):
     if ch == 2 and rng.uniform() < 0.4:
         pcm[:, 1] = 0.0
     rms = (0.05 + 0.2 * rng.uniform(size=(1, T))).astype(np.float32) if settings.get("normalize_volume") else None
-    r = refbind.RefSource({"display_mode": "waveform", **settings}, channels=ch)
-    ref = r.run_wave(pcm[0], T, hop, rms=None if rms is None else rms[0])
+    return settings, ch, hop, pcm, rms
+
+
+@pytest.mark.parametrize("seed", range(30))
+def test_wave_oracle_randomised_settings_bit_exact_vs_compiled_reference(seed, ref):
+    """Differential fuzz of the waveform-mode oracle against the unmodified reference: random width, window length, packet size,
+    channel layout, volume normalisation, stretches of zeros and of full-scale samples (the all-zero silent rule's raw material)."""
+    _check_bit_exact(ref[f"random{seed}"], *_random_case(seed))
+
+
+def _check_bit_exact(rec, settings, ch, hop, pcm, rms):
+    from oracle.oraclebind import OracleWave
+
+    assert digest(pcm) + digest(rms) == rec["inputs"], "inputs differ from the ones the reference was run on"
+    T = pcm.shape[-1] // hop
     out = OracleWave(settings, channels=ch).run(pcm[0], T, hop, rms=None if rms is None else rms[0])
-    assert np.array_equal(ref["out"], out["out"]), settings
-    assert np.array_equal(ref["silent"], out["silent"]), settings
+    assert digest(out["out"]) == rec["out"], settings
+    assert digest(out["silent"]) == rec["silent"], settings
+
+
+def reference_records():
+    """m_decibels and m_last_silent of the compiled reference (oracle/_ref) after every tick of each case above, as digests;
+    tests/golden/make_golden.py stores them."""
+    from oracle import refbind
+
+    recs = {}
+    for name, (settings, ch, hop, pcm, rms) in [(f"case{i}", (s, c, h) + _case(s, c, h, T=50)) for i, (s, c, h) in enumerate(WAVE_CASES)] \
+            + [(f"random{seed}", _random_case(seed)) for seed in range(30)]:
+        T = pcm.shape[-1] // hop
+        r = refbind.RefSource({"display_mode": "waveform", **settings}, channels=ch).run_wave(
+            pcm[0], T, hop, rms=None if rms is None else rms[0])
+        recs[name] = {"inputs": digest(pcm) + digest(rms), "out": digest(r["out"]), "silent": digest(r["silent"])}
+    return recs
 
 
 @pytest.mark.parametrize("path", GOLD, ids=[p.stem for p in GOLD])
